@@ -1,13 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- FEAR-XS per-frame inference throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (FEARNet.track + box decode) over one batch of synthetic
 crops: 256 search crops (3x256x256 fp32, ImageNet-normalised uniform uint8, seed 20260924) with
 their 256 template feature maps, per GPU (BASELINE config 2; at N GPUs each rank owns a contiguous
 256-frame shard of the 256*N batch -- config 4 at N=8 -- and the step ends with ONE all-gather of
 the 48-byte box records).  One JSON line on stdout (rank 0).  See DESIGN.md section "Measurement".
+
+--dump-outputs DIR writes the gathered box records of the last timed step (rank 0) as DIR/box_xywh.npy
+(float64, (N,4)), DIR/score.npy (float32, (N,)) and DIR/cell_row_col_flat.npy (float64, (N,3)); the inputs
+depend only on the seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -202,6 +206,16 @@ def parity_check(net, boxes_all, world, B, frames_per_rank=4):
             "oracle's (fp64) for the check"}
 
 
+def dump_outputs(out_dir, rec):
+    """The decoded FearBox records (``net.boxes_to_numpy``) as float64 / float32 .npy files."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"box_xywh": np.stack([rec[k] for k in ("x", "y", "w", "h")], 1),
+              "score": np.ascontiguousarray(rec["score"]),
+              "cell_row_col_flat": np.stack([rec[k] for k in ("row", "col", "flat")], 1).astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def read_video(path):
     import cv2
 
@@ -331,7 +345,13 @@ def main():
                     help="batch = BASELINE config 2/4 (default, the contract line); stream = config 3 only")
     ap.add_argument("--no-stream", action="store_true", help="skip the config-3 streaming measurement")
     ap.add_argument("--no-parity", action="store_true", help="skip the post-run oracle parity check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the box records of the last timed step as .npy files under DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "batch"):
+        ap.error("--dump-outputs applies to the batch workload of --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -423,17 +443,18 @@ def main():
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """(ms for ``steps`` calls of fn, what the last call returned)"""
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         sync_all()
         a.record(stream)
         for _ in range(steps):
-            fn()
+            out = fn()
         b.record(stream)
         sync_all()
         ms = torch.tensor([a.elapsed_time(b)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     clocks = ClockSampler(local_rank).__enter__()
     for _ in range(args.warmup):
@@ -441,7 +462,7 @@ def main():
     clocks.wait_first_sample()
     l0 = net.launch_count()
     clocks.begin()
-    ms_total = timed(step_device, args.steps)
+    ms_total, last_boxes = timed(step_device, args.steps)
     if ms_total < 400.0:  # keep the GPU under the same load until nvidia-smi (100 ms period) has sampled it
         extra = int(400.0 / (ms_total / args.steps)) + 1
         for _ in range(extra):
@@ -454,11 +475,11 @@ def main():
 
     for _ in range(args.warmup):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     fps_e2e = total * args.steps / (ms_e2e * 1e-3)
     for _ in range(args.warmup):
         step_e2e(x_host)
-    ms_e2e32 = timed(lambda: step_e2e(x_host), args.steps)
+    ms_e2e32, _ = timed(lambda: step_e2e(x_host), args.steps)
 
     # ---- per-stage device time over another K steps (CUDA events around every launch, same stream) ----
     net.profile(True)
@@ -521,6 +542,8 @@ def main():
     if rank == 0 and not args.no_parity:
         parity = parity_check(net, final_boxes, world, B)
         parity["e2e_records_identical"] = bool(torch.equal(final_boxes, final_boxes_e2e))
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, net.boxes_to_numpy(last_boxes))
     stream_line = None
     if rank == 0 and world == 1 and not args.no_stream:
         stream_line = run_stream(net, dev)

@@ -12,7 +12,8 @@ oracle restatement reproduces each of them bit-for-bit:
   on the synthetic crops, template batch B and 1;
 * ``tests/golden/train_step.npz``      -- FEARNet in train() mode (BatchNorm batch statistics): forward maps,
   gradient norms and the updated running statistics of one step (fear_lightning_model.py:60-62 calls
-  ``model.forward`` in training).
+  ``model.forward`` in training);
+* ``tests/golden/train_step_fp64.npz`` -- the gradient norms of the same step in float64.
 """
 import os
 
@@ -101,6 +102,21 @@ def train_step():
     print("train: loss", float(loss), "params with grad", len(grads))
 
 
+def train_step_fp64():
+    """The gradient norms of train_step() in float64.  In float32 the biases of convolutions that feed a train-mode
+    BatchNorm (exact gradient zero: the batch mean cancels them) carry rounding noise that differs between host CPUs."""
+    net = ref_shims.build_reference_net().double().train()
+    g = torch.Generator().manual_seed(5)
+    z = torch.randn(2, 3, 128, 128, generator=g).double()
+    x = torch.randn(2, 3, 256, 256, generator=g).double()
+    out = net((z, x))
+    (out[R].log().mean() + out[C].mean()).backward()
+    grads = {k: float(p.grad.norm()) for k, p in net.named_parameters() if p.grad is not None}
+    np.savez_compressed(os.path.join(OUT, "train_step_fp64.npz"), grad_names=np.array(sorted(grads)),
+                        grad_norms=np.array([grads[k] for k in sorted(grads)]))
+    print("train fp64: params with grad", len(grads))
+
+
 def main():
     torch.set_num_threads(os.cpu_count())
     net = ref_shims.build_reference_net()
@@ -108,6 +124,7 @@ def main():
     smooth(net, sd32)
     update_branch(fo.to_dtype(sd32, torch.float64))
     train_step()
+    train_step_fp64()
 
 
 if __name__ == "__main__":

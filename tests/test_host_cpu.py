@@ -65,7 +65,17 @@ def test_train_mode_forward_matches_reference_training_step():
     loss.backward()
     grads = {k: float(p.grad.norm()) for k, p in net.named_parameters() if p.grad is not None}
     assert sorted(grads) == g["grad_names"].tolist()
-    np.testing.assert_allclose([grads[k] for k in sorted(grads)], g["grad_norms"], rtol=2e-3, atol=1e-7)
+    # gradient norms in float64: in float32 the biases of convolutions that feed a train-mode BatchNorm (exact
+    # gradient zero) hold rounding noise that differs between host CPUs
+    g64 = np.load(os.path.join(GOLDEN, "train_step_fp64.npz"))
+    net64 = fb.FEARNet(**fb.FEAR_XS_MODEL_KWARGS)
+    net64.load_state_dict(load_full_state(), strict=True)
+    net64 = net64.double().train()
+    out64 = net64((z.double(), x.double()))
+    (out64[R].log().mean() + out64[C].mean()).backward()
+    grads64 = {k: float(p.grad.norm()) for k, p in net64.named_parameters() if p.grad is not None}
+    assert sorted(grads64) == g64["grad_names"].tolist() == g["grad_names"].tolist()
+    np.testing.assert_allclose([grads64[k] for k in sorted(grads64)], g64["grad_norms"], rtol=2e-3, atol=1e-7)
     sd = net.state_dict()
     for key in g.files:
         if key.startswith("bn__"):  # running statistics were updated with the batch statistics

@@ -1,14 +1,11 @@
 """CPU tests: the oracle restatement against the golden vectors recorded from the reference's
-own source (oracle/make_golden.py), and -- when /root/reference is present -- against the
-reference itself."""
+own source (oracle/make_golden*.py)."""
 import hashlib
 
 import numpy as np
-import pytest
 import torch
 
 from oracle import fear_oracle as fo
-from oracle import ref_shims
 from tests.helpers import assert_maps_close, golden, load_full_state
 
 R, C = fo.TARGET_REGRESSION_LABEL_KEY, fo.TARGET_CLASSIFICATION_KEY
@@ -129,15 +126,19 @@ def test_smooth_tracker_prefix_trajectory(state_dict, golden_dir):
         assert list(trk.update(frames[i])["bbox"]) == g["trajectory"][i - 1].tolist(), i
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="/root/reference not present (GPU box)")
 def test_restatement_equals_reference_source(state_dict):
-    """Build container only: oracle == the reference's own FEARNet, bit-for-bit (fp32)."""
-    net = ref_shims.build_reference_net()
-    sd = fo.load_lightning_state(ref_shims.REF_CKPT)
-    for k, v in state_dict.items():
-        assert torch.equal(sd[k], v), k
+    """oracle == the reference's own FEARNet on the seed-7 crops, against its outputs recorded by
+    oracle/make_golden_restatement.py (which also asserts bit-equality where it runs).  The weight fixture must be
+    the checkpoint byte for byte.  fp64 maps to rounding level; fp32 maps within the noise of another host CPU's
+    kernels (measured 2e-6 inf-norm, 1.2e-4 element-wise between AVX-512 and AVX2)."""
+    g = golden("restatement_seed7.npz")
+    assert sorted(state_dict) == g["keys"].tolist()
+    for k, digest in zip(g["keys"], g["sha256"]):
+        assert hashlib.sha256(state_dict[k].contiguous().numpy().tobytes()).hexdigest() == digest, k
     zt, xt, _, _ = fo.synthetic_crops(2, seed=7)
-    with torch.no_grad():
-        ref = net((zt, xt))
+    mine = fo.forward(fo.to_dtype(state_dict, torch.float64), zt.double(), xt.double())
+    np.testing.assert_allclose(mine[R].numpy(), g["reg64"], rtol=1e-10)
+    np.testing.assert_allclose(mine[C].numpy(), g["cls64"], rtol=1e-9, atol=1e-11)
     mine = fo.forward(state_dict, zt, xt)
-    assert torch.equal(ref[R], mine[R]) and torch.equal(ref[C], mine[C])
+    assert_maps_close(mine[R].numpy(), g["reg32"], "reg fp32", inf_tol=1e-5)
+    assert_maps_close(mine[C].numpy(), g["cls32"], "cls fp32", inf_tol=1e-5)
