@@ -4,6 +4,7 @@ from .constants import TARGET_CLASSIFICATION_KEY, TARGET_REGRESSION_LABEL_KEY  #
 from .fear_net import FEARNet  # noqa: F401
 from .box_coder import FEARBoxCoder, TrackerDecodeResult  # noqa: F401
 from .tracker import FEARTracker, Tracker, TrackingState  # noqa: F401
+from .multi_tracker import FEARMultiTracker  # noqa: F401
 
 FEAR_XS_MODEL_KWARGS = dict(  # reference model_training/config/model/fear.yaml
     backbone="custom_fbnet", img_size=256, pretrained=True, stride=2, conv_block="sep_conv", towernum=2, mobile=True,

@@ -25,6 +25,23 @@ BOX_DTYPE = np.dtype(
 )
 assert BOX_DTYPE.itemsize == ctypes.sizeof(FearBox) == 48
 
+
+class FearFrame(ctypes.Structure):
+    _fields_ = [("data", c_uint64), ("h", c_int32), ("w", c_int32)]
+
+
+FRAME_DTYPE = np.dtype([("data", "<u8"), ("h", "<i4"), ("w", "<i4")])
+assert FRAME_DTYPE.itemsize == ctypes.sizeof(FearFrame) == 16
+
+
+class FearTrack(ctypes.Structure):
+    _fields_ = [(name, c_int32) for name in ("x", "y", "w", "h", "cx", "cy", "cw", "ch", "pad_r", "pad_g", "pad_b",
+                                             "reserved")]
+
+
+TRACK_DTYPE = np.dtype([(name, "<i4") for name, _ in FearTrack._fields_])
+assert TRACK_DTYPE.itemsize == ctypes.sizeof(FearTrack) == 48
+
 _SIGNATURES = {
     # name: (restype, argtypes)
     "fear_init": (c_int, [c_int]),
@@ -45,6 +62,8 @@ _SIGNATURES = {
     "fear_get_features_u8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "fear_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     "fear_crop_resize_u8": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]),
+    "fear_track_crops_u8": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_double, c_void_p, c_void_p]),
+    "fear_track_advance": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "fear_decode": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "fear_corr_concat_f32": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "fear_corr_concat_workspace_bytes": (c_size_t, [c_int, c_int]),

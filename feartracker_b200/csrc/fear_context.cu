@@ -17,6 +17,7 @@
 #include "kernels_stem_fused.cuh"
 #include "kernels_irf_fused.cuh"
 #include "kernels_dwpw_small.cuh"
+#include "kernels_multitrack.cuh"
 
 using namespace fear;
 
@@ -1022,6 +1023,29 @@ extern "C" int fear_crop_resize_u8(const uint8_t* d_frame, int H, int W, const i
   const int n = out_size * out_size;
   crop_resize_u8_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(d_frame, H, W, d_params, d_crop, out_size);
   return check_launch("crop_resize_u8_kernel");
+}
+
+// N context crops for N tracks in one launch, context boxes and resize coefficients derived on the device from the
+// tracks' boxes (kernels_multitrack.cuh).
+extern "C" int fear_track_crops_u8(const FearFrame* d_frames, int F, const int32_t* d_frame_of_track, FearTrack* d_tracks,
+                                   int N, int out_size, double context, uint8_t* d_crops, void* stream) {
+  if (!d_frames || !d_frame_of_track || !d_tracks || !d_crops || F < 1 || N < 1 || N > 65535 || out_size < 1 ||
+      out_size > 1024 || !(context >= 0.0 && context <= 1e6))
+    return set_err(FEAR_EINVAL, "bad argument");
+  const dim3 grid((out_size * out_size + 255) / 256, N);
+  track_crops_u8_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_frames, F, d_frame_of_track, d_tracks, out_size,
+                                                                context, d_crops);
+  return check_launch("track_crops_u8_kernel");
+}
+
+// Decoded box records -> next box of every live track (rescale_bbox + clamp_bbox on the device).
+extern "C" int fear_track_advance(const FearBox* d_boxes, const FearFrame* d_frames, const int32_t* d_frame_of_track,
+                                  FearTrack* d_tracks, int N, int instance_size, void* stream) {
+  if (!d_boxes || !d_frames || !d_frame_of_track || !d_tracks || N < 1 || instance_size < 1)
+    return set_err(FEAR_EINVAL, "bad argument");
+  track_advance_kernel<<<(N + 127) / 128, 128, 0, (cudaStream_t)stream>>>(d_boxes, d_frames, d_frame_of_track,
+                                                                           d_tracks, N, instance_size);
+  return check_launch("track_advance_kernel");
 }
 
 extern "C" int fear_decode(const float* d_bbox, const float* d_cls, int B, int apply_sigmoid, FearBox* d_boxes,

@@ -390,20 +390,13 @@ __global__ void __launch_bounds__(256) gemm_nt_ffma_kernel(const float* __restri
 // `params`:  [0..3] context x, y, w, h (frame coordinates, may leave the frame); [4..6] padding colour RGB; [7] unused;
 // then xofs[S], xa0[S], xa1[S], yofs[S], ya0[S], ya1[S] for an S x S output.  out: [S][S][3] uint8 (HWC).
 // ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) crop_resize_u8_kernel(const uint8_t* __restrict__ frame, int H, int W,
-                                                             const int* __restrict__ params, uint8_t* __restrict__ out,
-                                                             int S) {
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= S * S) return;
-  const int dy = idx / S, dx = idx - dy * S;
-  const int cx = __ldg(params), cy = __ldg(params + 1), cw = __ldg(params + 2), ch = __ldg(params + 3);
-  const int* tx = params + 8;
-  const int* ty = params + 8 + 3 * S;
-  const int x0 = __ldg(tx + dx), a0 = __ldg(tx + S + dx), a1 = __ldg(tx + 2 * S + dx);
-  const int yo = __ldg(ty + dy), b0 = __ldg(ty + S + dy), b1 = __ldg(ty + 2 * S + dy);
+// One output pixel (all three channels) of the padded, resized context window (cx, cy, cw, ch): x0 / a0 / a1 are the
+// column's source offset and coefficients, yo / b0 / b1 the row's.  Shared with track_crops_u8_kernel.
+__device__ __forceinline__ void crop_resize_pixel(const uint8_t* __restrict__ frame, int H, int W, int cx, int cy,
+                                                  int cw, int ch, const int (&pad)[3], int x0, int a0, int a1, int yo,
+                                                  int b0, int b1, uint8_t* __restrict__ out_px) {
   const int x1 = min(x0 + 1, cw - 1);
   const int y0 = min(max(yo, 0), ch - 1), y1 = min(max(yo + 1, 0), ch - 1);
-  int pad[3] = {__ldg(params + 4), __ldg(params + 5), __ldg(params + 6)};
   auto px = [&](int y, int x, int c) -> int {  // padded context window
     const int fy = cy + y, fx = cx + x;
     return (fy >= 0 && fy < H && fx >= 0 && fx < W) ? (int)__ldg(frame + ((long long)fy * W + fx) * 3 + c) : pad[c];
@@ -413,8 +406,22 @@ __global__ void __launch_bounds__(256) crop_resize_u8_kernel(const uint8_t* __re
     const int s0 = px(y0, x0, c) * a0 + px(y0, x1, c) * a1;
     const int s1 = px(y1, x0, c) * a0 + px(y1, x1, c) * a1;
     const int v = (((b0 * (s0 >> 4)) >> 16) + ((b1 * (s1 >> 4)) >> 16) + 2) >> 2;
-    out[(long long)idx * 3 + c] = (uint8_t)min(max(v, 0), 255);
+    out_px[c] = (uint8_t)min(max(v, 0), 255);
   }
+}
+
+__global__ void __launch_bounds__(256) crop_resize_u8_kernel(const uint8_t* __restrict__ frame, int H, int W,
+                                                             const int* __restrict__ params, uint8_t* __restrict__ out,
+                                                             int S) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= S * S) return;
+  const int dy = idx / S, dx = idx - dy * S;
+  const int cx = __ldg(params), cy = __ldg(params + 1), cw = __ldg(params + 2), ch = __ldg(params + 3);
+  const int* tx = params + 8;
+  const int* ty = params + 8 + 3 * S;
+  const int pad[3] = {__ldg(params + 4), __ldg(params + 5), __ldg(params + 6)};
+  crop_resize_pixel(frame, H, W, cx, cy, cw, ch, pad, __ldg(tx + dx), __ldg(tx + S + dx), __ldg(tx + 2 * S + dx),
+                    __ldg(ty + dy), __ldg(ty + S + dy), __ldg(ty + 2 * S + dy), out + (long long)idx * 3);
 }
 
 // ------------------------------------------------------------------------------------------

@@ -18,6 +18,8 @@
  *
  *   fear_head_update      BoxTower.forward(search, kernel, update)   blocks.py:174-179
  *   fear_crop_resize_u8   get_extended_crop (crop + pad + resize)    model_training/utils/utils.py:215-253
+ *   fear_track_crops_u8   the same for N tracks at once, context box computed on the device
+ *   fear_track_advance    Tracker._rescale_bbox + clamp_bbox of FEARTracker.update, on the device
  *
  * Conventions: every pointer named d_* is a DEVICE pointer owned by the caller (torch keeps
  * ownership); tensors are dense fp32 in the reference's NCHW layout unless stated; `stream`
@@ -130,6 +132,34 @@ int fear_forward(FearContext* h, const float* d_template, const float* d_search,
  * cv::resize computes them (feartracker_b200.image_ops.resize_tables). */
 int fear_crop_resize_u8(const uint8_t* d_frame, int H, int W, const int32_t* d_params, uint8_t* d_crop, int out_size,
                         void* stream);
+
+/* ---- batched tracking loop with device-resident state ---------------------------------
+ * One input frame of a step: absolute device pointer, so a captured CUDA graph stays valid whatever buffer the
+ * frame sits in. */
+typedef struct FearFrame {
+  const uint8_t* data; /* DEVICE pointer to (h, w, 3) RGB uint8, row-major                   */
+  int32_t h, w;
+} FearFrame;
+
+/* Device-resident state of one target (FEARTracker.tracking_state). */
+typedef struct FearTrack {
+  int32_t x, y, w, h;                    /* current box in frame pixels (tracking_state.bbox)          */
+  int32_t cx, cy, cw, ch;                /* context box of the last crop (tracking_state.mapping)      */
+  int32_t pad_r, pad_g, pad_b, reserved; /* rint(mean colour of the init frame), clipped to 0..255     */
+} FearTrack;
+
+/* For every track n with d_frame_of_track[n] in [0, F): context box of (x, y, w, h) grown by `context` per side
+ * (image_ops.context_box), stored into the track's cx..ch, and crop n of d_crops (N, out_size, out_size, 3) cut from
+ * frame d_frames[d_frame_of_track[n]] -- bit-identical to fear_crop_resize_u8 with the host's crop_params (and so to
+ * cv2).  Tracks with index -1 are skipped (their crop and state are left untouched).  Search crops: out_size 256,
+ * context = search_context; template crops: 128, template_bbox_offset. */
+int fear_track_crops_u8(const FearFrame* d_frames, int F, const int32_t* d_frame_of_track, FearTrack* d_tracks, int N,
+                        int out_size, double context, uint8_t* d_crops, void* stream);
+/* For every track n with d_frame_of_track[n] >= 0: box = clamp_bbox(rescale_bbox(d_boxes[n], (cx, cy, cw, ch),
+ * instance_size), frame size of d_frames[d_frame_of_track[n]]) bit for bit (image_ops), written into x..h.
+ * Frame indices are not bounds-checked here: pass the table fear_track_crops_u8 accepted. */
+int fear_track_advance(const FearBox* d_boxes, const FearFrame* d_frames, const int32_t* d_frame_of_track,
+                       FearTrack* d_tracks, int N, int instance_size, void* stream);
 
 /* Decode maps produced elsewhere: bbox (B,4,16,16), cls logits (B,1,16,16) -> boxes[B].
  * apply_sigmoid = 0 treats cls as already-activated scores (decode(use_sigmoid=False)). */
